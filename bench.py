@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RAO solves/s of the B200-native hot path (BASELINE.json metric), one JSON line on rank 0.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg2|cfg3|cfg3q|sweep]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg2|cfg3|cfg3q|sweep] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (Model.solveDynamics for every (design, case) unit of the batch:
 excitation tables, drag-linearisation fixed-point loop, 6x6 complex impedance solve per frequency).
@@ -16,6 +16,13 @@ workload sweep (BASELINE.json configs[3] shard): 1250 VolturnUS-S geometry varia
 
 value = units of all ranks / max-over-ranks device time (CUDA events, inputs resident in HBM).
 e2e   = same metric through the host-buffer C-ABI call (pinned host inputs -> H2D -> kernels -> D2H).
+
+--dump-outputs DIR writes what the last timed step returned (Xi, status, ... of every unit) as DIR/<name>.npy in float64,
+complex arrays as <name>_real / <name>_imag; inputs are seeded, so two builds can be compared output for output.  One GPU:
+every output of the session (Xi, status, B_drag, and F_2nd / F_2nd_mean for cfg3q); N > 1: Xi and status of all ranks'
+units, whichever exchange ran.  It covers the solveDynamics path of workloads cfg2, cfg3, cfg3q and sweep; the farm and
+flex workloads (bench_extra.py) and --impl reference (the CPU checker, not this project's code) refuse it.
+bench.py writes nothing into the tree, which may be read-only.
 """
 import argparse
 import json
@@ -29,9 +36,11 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # no __pycache__ in the tree
 
 METRIC = "RAO solves/sec (freq-bins x cases x designs)"
 UNIT = "solves/s"
+DUMP_LIMIT = 60 << 20                   # bytes of --dump-outputs in all (< 64 MB)
 
 
 def sea_states(seed, n):
@@ -281,6 +290,31 @@ def parity_block(designs, cs, Xi, status, max_designs=8):
                 checker="oracle/raft_oracle.c (pinned to reference pickles and reference runs: tests/test_oracle_golden.py)")
 
 
+def sample_outputs(outs, limit=DUMP_LIMIT):
+    """Host float64 copies of one step's outputs for --dump-outputs: complex arrays split into <name>_real / <name>_imag,
+    integer arrays converted.  Every array leads with the (design, case) unit axes.  Past ``limit`` bytes in all, a fixed
+    seeded sample of units is kept, the same units in every array (flattened unit axis), listed in ``sample_units``."""
+    import torch
+    t0 = next(iter(outs.values()))
+    n_units = t0.shape[0] * t0.shape[1]
+    per_unit = sum(t[0, 0].numel() * (16 if t.is_complex() else 8) for t in outs.values()) + 8
+    keep = None
+    if per_unit * n_units > limit:
+        keep = np.sort(np.random.default_rng(0).choice(n_units, limit // per_unit, replace=False))
+    res = {}
+    for k, t in outs.items():
+        if keep is not None:
+            t = t.flatten(0, 1)[torch.as_tensor(keep, device=t.device)]
+        a = t.cpu().numpy()
+        if np.iscomplexobj(a):
+            res[k + "_real"], res[k + "_imag"] = a.real.astype(np.float64), a.imag.astype(np.float64)
+        else:
+            res[k] = a.astype(np.float64)
+    if keep is not None:
+        res["sample_units"] = keep.astype(np.float64)
+    return res
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU implementation of the path on the box's host cores.  Two numbers:
     the pinned C oracle port with all host threads (the STRONG CPU figure: value of the line) and, when
@@ -352,7 +386,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained-load and sweep-shard extra keys")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64; a seeded sample of units past 60 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("farm", "flex")):
+        ap.error("--dump-outputs covers the solveDynamics path of workloads cfg2, cfg3, cfg3q and sweep")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -478,6 +518,20 @@ def measure(args, designs, cs, cfg, rank, world, dev, full):
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
     launches = solver.launch_count() - launches0
+    dump = None
+    if args.dump_outputs and full:
+        # now: the roofline solves below write the same buffers again.  At N > 1 the caller receives every rank's units;
+        # both exchanges give Xi and status of all of them (the NCCL one gathers status here, outside the timed steps)
+        if sh is not None:
+            outs = dict(Xi=last["g"].flatten(0, 1), status=last["s"].flatten(0, 1))
+        elif world > 1:
+            st_all = torch.empty((world,) + tuple(sess.out["status"].shape), dtype=torch.int32, device=dev)
+            dist.all_gather_into_tensor(st_all, sess.out["status"])
+            outs = dict(Xi=gathered.flatten(0, 1), status=st_all.flatten(0, 1))
+        else:
+            outs = sess.out
+        if rank == 0:
+            dump = sample_outputs(outs)
     clocks = sampler.stop() if sampler.run or not sampler.ok else dict(sm_mhz=None, sm_max_mhz=sampler.max_mhz, reasons=["sampler disabled (diagnostic run)"], samples=0)
     ms = sum(a.elapsed_time(b) for a, b in ev)
     t_ms = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -661,6 +715,10 @@ def measure(args, designs, cs, cfg, rank, world, dev, full):
             line["per_rank"] = per_rank
         if sustained is not None:
             line["sustained"] = sustained
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), a)
     if sh is not None:
         torch.cuda.synchronize()
         dist.barrier()

@@ -3,9 +3,12 @@
 TEST INFRASTRUCTURE ONLY -- importable from tests/, __graft_entry__.smoke() and bench.py's
 cpu_baseline / --impl reference legs.  The product package ``raft_b200`` never imports this.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -63,13 +66,29 @@ def _qs_struct(P, keep):
     return q
 
 
+_tmp_lib = None
+
+
 def build(force=False):
-    """Compile the C oracle with gcc (no -march flags: plain IEEE double, no FMA contraction)."""
-    os.makedirs(os.path.dirname(LIB), exist_ok=True)
-    if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(SRC):
+    """Compile the C oracle with gcc (no -march flags: plain IEEE double, no FMA contraction) into oracle/_build, or
+    into a fresh temporary directory when the tree is read-only (bench.py may run from one)."""
+    global _tmp_lib
+    lib = LIB
+    if force or not os.path.exists(lib) or os.path.getmtime(lib) < os.path.getmtime(SRC):
+        if _tmp_lib is not None and not force:
+            return _tmp_lib
+        try:
+            os.makedirs(os.path.dirname(lib), exist_ok=True)
+            writable = os.access(os.path.dirname(lib), os.W_OK)
+        except OSError:
+            writable = False
+        if not writable:
+            tmp = tempfile.mkdtemp(prefix="raft_oracle_")
+            atexit.register(shutil.rmtree, tmp, True)          # the mapped library outlives its file
+            lib = _tmp_lib = os.path.join(tmp, os.path.basename(LIB))
         subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-fopenmp", "-ffp-contract=off",
-                               "-o", LIB, SRC, "-lm"])
-    return LIB
+                               "-o", lib, SRC, "-lm"])
+    return lib
 
 
 _lib = None

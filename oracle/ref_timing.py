@@ -1,7 +1,7 @@
 """CPU baseline leg: the UNMODIFIED Python reference timed on this box's host cores (BASELINE.md 4.1-4.3).
 
 TEST / MEASUREMENT INFRASTRUCTURE ONLY (bench.py's cpu_baseline and ``--impl reference``).  The reference is the pip
-install under baseline/_ref (baseline/install_reference.py; git-ignored, shipped to the GPU box), imported through
+install under oracle/_ref (oracle/make_ref.py; git-ignored, shipped to the GPU box), imported through
 oracle/ref_harness.py's stubs exactly as when the goldens were made: turbine + mooring stripped, zero mean offset,
 C_moor = diag(7e4, 7e4, 0, 0, 0, 1.2e8).  Timed: wall clock around ``Model.solveDynamics`` only (model construction
 excluded), one sea state of the workload's seeded table per call; single process (the reference is single-threaded)
@@ -15,9 +15,9 @@ import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(HERE, "_ref")
 
-# workload -> (design file under baseline/_ref/inputs, nw, max_freq [Hz], sea-state seed, potModMaster override)
+# workload -> (design file under oracle/_ref/inputs, nw, max_freq [Hz], sea-state seed, potModMaster override)
 CONFIGS = {
     "cfg1": ("designs/OC3spar.yaml", None, None, None, None),
     "cfg2": ("designs/VolturnUS-S.yaml", 1024, 0.512, 2, 1),
@@ -64,7 +64,7 @@ def _worker(name, first_case, n_cases, budget_s):
 
 
 def _spawn(name, first_case, n_cases, budget_s):
-    env = dict(os.environ, OMP_NUM_THREADS="1", OPENBLAS_NUM_THREADS="1", MKL_NUM_THREADS="1")
+    env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1", OMP_NUM_THREADS="1", OPENBLAS_NUM_THREADS="1", MKL_NUM_THREADS="1")
     return subprocess.Popen([sys.executable, os.path.abspath(__file__), "--worker", name, str(first_case), str(n_cases), str(budget_s)],
                             stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env, cwd=ROOT)
 
@@ -88,9 +88,9 @@ def _collect(procs, timeout):
 def measure(workload="cfg2", budget_s=20.0, processes=None):
     """-> dict for the JSON line: solves/s of the unmodified reference, 1 process and P processes, on a bounded sample."""
     if not available():
-        return dict(unavailable="baseline/_ref not installed (run baseline/install_reference.py in the build container)")
+        return dict(unavailable="oracle/_ref not installed (build() where the reference source tree is present, or oracle/make_ref.py)")
     name = workload if workload in CONFIGS else "cfg2"
-    res = dict(kind="reference", code="unmodified WISDEM/RAFT (pip-installed under baseline/_ref), moorpy/ccblade/pyhams/matplotlib import lines stubbed",
+    res = dict(kind="reference", code="unmodified WISDEM/RAFT (pip-installed under oracle/_ref), moorpy/ccblade/pyhams/matplotlib import lines stubbed",
                timed="Model.solveDynamics wall clock, model construction excluded")
     one = _collect([_spawn("cfg1", 0, 1, budget_s)], timeout=120)[0]
     if "error" not in one:

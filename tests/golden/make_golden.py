@@ -31,6 +31,18 @@ REF = rh.REF_ROOT
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
+def savez_lzma(path, **arrays):
+    """np.savez with LZMA-compressed members (zip method 14; np.load reads it as is): the fixtures holding large
+    float64 tables stay under 1 MB, where deflate would leave them at 2-3 MB."""
+    import io
+    import zipfile
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as zf:
+        for k, v in arrays.items():
+            b = io.BytesIO()
+            np.lib.format.write_array(b, np.asanyarray(v), allow_pickle=False)
+            zf.writestr(k + ".npy", b.getvalue())
+
+
 def seeded_cases(seed, n):
     """SURVEY.md 8d sea-state distribution: Hs~U[1,10], Tp~U[5,18], gamma=0 (IEC auto), beta~U[-180,180)."""
     rng = np.random.default_rng(seed)
@@ -336,7 +348,7 @@ def fixture_flexible(name, yaml_path, pickles):
     out["n_iter"], out["xi_start"] = np.int32(int(model.nIter)), np.float64(model.XiStart)
     out["ref_run_solve_cases"], out["ref_run_solve_Xi"], out["ref_run_solve_passes"] = np.array(cases), np.array(Xi), np.array(passes, dtype=np.int32)
     path = os.path.join(OUT, name + ".npz")
-    np.savez_compressed(path, **out)
+    savez_lzma(path, **out)
     print("%-28s nDOF=%3d Ns=%3d  %.1f s  %.0f KB" % (name, int(P["gen_nDOF"]), len(P["node_ls"]), time.time() - t0, os.path.getsize(path) / 1024))
 
 
@@ -450,8 +462,8 @@ def main():
         A, B, w1 = bem.read_wamit1(hp + ".1")
         _, _, Re, Im, w3, heads = bem.read_wamit3(hp + ".3")
         qtf_rows = np.loadtxt(hp + ".12d")                  # raw .12d rows, for the QTF reader test off the build box
-        np.savez_compressed(os.path.join(OUT, "wamit_marin_semi.npz"), A=A, B=B, w1=w1, Re=Re.astype(np.float64),
-                            Im=Im.astype(np.float64), w3=w3, heads=heads, qtf_rows=qtf_rows.astype(np.float32))
+        savez_lzma(os.path.join(OUT, "wamit_marin_semi.npz"), A=A, B=B, w1=w1, Re=Re.astype(np.float64),
+                   Im=Im.astype(np.float64), w3=w3, heads=heads, qtf_rows=qtf_rows.astype(np.float32))
         print("wamit_marin_semi.npz %.0f KB" % (os.path.getsize(os.path.join(OUT, "wamit_marin_semi.npz")) / 1024))
     import json
     dj = os.path.join(OUT, "designs.json")
