@@ -309,13 +309,65 @@ def solve_dynamics(batch, cases, n_iter=10, tol=0.01, xi_start=0.0, cluster_size
     check(lib.raftk_solve_dynamics_host(C.byref(d), C.byref(c), C.byref(o), C.byref(os_)))
     if np.any(outs["status"][..., 2] & FLAG_PLAN):
         # the device deduplicated more distinct node spacings than the host-side hint allowed for (near-tolerance
-        # chains): those units ran no pass and hold zeros.  Re-run with worst-case table sizes (hint 0).
+        # chains): those units ran no pass and hold zeros.  Re-run with the table sizes the device's own class numbering
+        # needs: the same kernel as a correctly hinted call (worst-case sizes, hint 0, rarely fit on chip, and the v1 solver
+        # they would fall back to refuses wave trains and Xi_init / Xi_last).  Hint 0 stays as the last resort.
         d = batch.struct(_host_ptr(batch.arrays))                 # a private copy: the cached struct keeps the hints
-        d.max_w_classes = d.max_h_classes = d.max_z_classes = 0
+        d.max_w_classes, d.max_h_classes, d.max_z_classes = device_step_classes(batch)
         check(lib.raftk_solve_dynamics_host(C.byref(d), C.byref(c), C.byref(o), C.byref(os_)))
+        if np.any(outs["status"][..., 2] & FLAG_PLAN):
+            d.max_w_classes = d.max_h_classes = d.max_z_classes = 0
+            check(lib.raftk_solve_dynamics_host(C.byref(d), C.byref(c), C.byref(o), C.byref(os_)))
         if np.any(outs["status"][..., 2] & FLAG_PLAN):
             raise _lib.RaftkError("step-class tables overflowed even with worst-case sizes")
     return outs
+
+
+def _first_match(close):
+    """Row j of the boolean matrix ``close`` [n, n] -> index of its first True among columns x < j, else j."""
+    n = len(close)
+    c = close & np.tri(n, k=-1, dtype=bool)
+    return np.where(c.any(axis=1), c.argmax(axis=1), np.arange(n))
+
+
+def device_step_classes(batch):
+    """Step-class table sizes (max_w, max_h, max_z) that the fused kernels' class numbering needs for every design of
+    ``batch``, restating its rule (raftk_fused.cuh / raftk_fused2.cuh k_fused_plan): a node's representative is the FIRST
+    earlier node whose spacing key lies within the tolerance, and its class is the number of representatives before that
+    node -- along a near-tolerance chain that can exceed the number of distinct keys the host-side hint counts."""
+    a = batch.arrays
+    mo, ms, fr, rA, ls = a["member_offset"], a["mem_node_start"], a["mem_frame"], a["mem_rA"], a["node_ls"]
+    need = [1, 1, 1]
+    for dd in range(batch.n_designs):
+        m0, m1 = int(mo[dd]), int(mo[dd + 1])
+        if m1 == m0:
+            continue
+        nb, ne = int(ms[m0]), int(ms[m1])
+        k = np.zeros([ne - nb, 3])
+        z0 = np.zeros(m1 - m0)
+        for m in range(m0, m1):
+            j0, j1 = int(ms[m]) - nb, int(ms[m + 1]) - nb
+            if j1 > j0:
+                z0[m - m0] = rA[m, 2] + ls[nb + j0] * fr[m, 2]
+                step = ls[nb + j0 + 1:nb + j1] - ls[nb + j0:nb + j1 - 1]
+                k[j0 + 1:j1] = fr[m, :3][None, :] * step[:, None]
+        for cols, tol in (((0, 1), 1e-11 * (np.abs(k[:, 0]) + np.abs(k[:, 1]))), ((2,), 1e-11 * np.abs(k[:, 2]))):
+            valid = np.any(np.abs(k[:, cols]) > 1e-14, axis=1)
+            if not valid.any():
+                continue
+            close = np.ones((len(k), len(k)), dtype=bool)
+            for col in cols:
+                close &= np.abs(k[None, :, col] - k[:, None, col]) <= tol[:, None]
+            rep = _first_match(close)
+            isrep = valid & (rep == np.arange(len(k)))
+            before = np.concatenate([[0], np.cumsum(isrep)])            # representatives before index x
+            slot = 0 if cols == (0, 1) else 1
+            need[slot] = max(need[slot], int(before[rep[valid]].max()) + 1)
+        close = np.abs(z0[None, :] - z0[:, None]) <= 1e-12 * np.maximum(1.0, np.abs(z0))[:, None]
+        rep = _first_match(close)
+        before = np.concatenate([[0], np.cumsum(rep == np.arange(len(z0)))])
+        need[2] = max(need[2], int(before[rep].max()) + 1)
+    return tuple(need)
 
 
 def solve_dynamics_farm(batch, cases, C_arr=None, M_arr=None, B_arr=None, n_iter=10, tol=0.01, xi_start=0.0, cluster_size=0,

@@ -133,7 +133,9 @@ def test_design_batch_and_device_session(solver, oracle):
     torch.cuda.synchronize()
     assert np.array_equal(dev["Xi"].cpu().numpy(), host["Xi"])
     assert np.array_equal(dev["status"].cpu().numpy(), host["status"])
-    # a workspace smaller than the batch forces design chunking: same answer
+    # a session with half the workspace: the fused solver has no design chunks (at 96 bins the smaller workspace only decides
+    # whether F0 may live there) and must give the same answer; the v1 solver's design-chunk loop is pinned in
+    # tests/test_dispatch_paths.py::test_v1_forced_design_batch_and_chunk_loop
     small = solver.DeviceSession(batch, solver.CaseTable(cs), workspace_bytes=sess.workspace_bytes // 2)
     dev2 = small.solve(n_iter=10)
     torch.cuda.synchronize()
