@@ -479,8 +479,11 @@ static int run_fused2(const raftk_designs *d, const raftk_cases *c, const raftk_
         k_fused_plan<<<d->n_designs, 128, psm, st>>>(D, plan, pl.blob, pl.maxW, pl.maxH, pl.maxZ, pl.nwl);
         g_launches++;
     }
-    static SmemOptIn opt;
-    CUDA_TRY(opt.ensure(k_rao_fused2, pl.smem));
+    // the lean instantiation unless the call needs a path it compiles out (see k_rao_fused2)
+    const bool full = d->A_w || d->B_w || out->F_drag || out->Xi_last || c->primary;
+    auto kern = full ? k_rao_fused2<true> : k_rao_fused2<false>;
+    static SmemOptIn opt_full, opt_lean;
+    CUDA_TRY((full ? opt_full : opt_lean).ensure(kern, pl.smem));
     const int units = d->n_designs * c->n_cases;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
@@ -498,7 +501,7 @@ static int run_fused2(const raftk_designs *d, const raftk_cases *c, const raftk_
         P.phase = c->primary ? phase : -1;
         {
             ProfScope ps(st, 2);
-            CUDA_TRY(cudaLaunchKernelEx(&cfg, k_rao_fused2, D, C, P));
+            CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, D, C, P));
         }
         g_launches++;
     }

@@ -19,8 +19,8 @@
 #define F2_TRW 8                 // values per round of the transposed warp reduction
 
 struct PlanLayout {
-    int o_mem, o_node, nstr, o_mat, o_wkey, o_hkey, o_zkey, o_int, total;      // offsets / sizes in doubles
-    int i_imem, i_nodew, i_nodeh, i_nodem, i_cnt, i_chunk, n_int;               // offsets in ints from o_int
+    int o_mem, o_node, nstr, o_mat, o_wkey, o_hkey, o_zkey, o_rec, o_int, total;   // offsets / sizes in doubles
+    int i_imem, i_nodem, i_cnt, i_chunk, n_int;                                    // offsets in ints from o_int
 };
 
 __host__ __device__ inline PlanLayout plan_layout(int NmP, int NsP, int maxW, int maxH, int maxZ)
@@ -35,11 +35,10 @@ __host__ __device__ inline PlanLayout plan_layout(int NmP, int NsP, int maxW, in
     L.o_hkey = p; p += maxH;
     L.o_zkey = p; p += maxZ;
     p = (p + 1) & ~1;
+    L.o_rec = p; p += 2 * (NsP + 12);          // node records {ls, factor-table offsets}; +12: the node walk prefetches up to 10 entries ahead
     L.o_int = p;
     int q = 0;
     L.i_imem = q; q += NmP * IMEM_STRIDE;
-    L.i_nodew = q; q += NsP + 12;              // +12: the node walk prefetches up to 10 entries ahead
-    L.i_nodeh = q; q += NsP + 12;
     L.i_nodem = q; q += NsP + 12;
     L.i_cnt = q; q += 4;                       // nW, nH, overflow, nZ
     L.i_chunk = q; q += 2 * ((NsP + CHUNK_NODES - 1) / CHUNK_NODES);   // per chunk of the RMS walk: direction mask, reduction-round mask
@@ -66,7 +65,8 @@ __global__ void __launch_bounds__(128) k_fused_plan(DesignsDev D, double *plan, 
     double *mem = blob + L.o_mem, *node = blob + L.o_node, *mat = blob + L.o_mat;
     double *wkey = blob + L.o_wkey, *hkey = blob + L.o_hkey, *zkey = blob + L.o_zkey;
     int *ib = reinterpret_cast<int *>(blob + L.o_int);
-    int *imem = ib + L.i_imem, *node_w = ib + L.i_nodew, *node_h = ib + L.i_nodeh, *node_m = ib + L.i_nodem, *cnt_g = ib + L.i_cnt;
+    int *imem = ib + L.i_imem, *node_m = ib + L.i_nodem, *cnt_g = ib + L.i_cnt;
+    double2 *rec = reinterpret_cast<double2 *>(blob + L.o_rec);
     double *scr = smem_raw;                                   // 3 * NsP key components
     double *z0s = scr + 3 * (size_t)NsP;                      // NmP first-node depths
     int *iscr = reinterpret_cast<int *>(z0s + NmP);           // 2 * NsP representatives
@@ -146,7 +146,9 @@ __global__ void __launch_bounds__(128) k_fused_plan(DesignsDev D, double *plan, 
         iscr[j] = rw; iscr[NsP + j] = rh;
     }
     __syncthreads();
-    // C: class id = rank of the representative among representatives; offsets into the factor tables (class * nwl)
+    // C: class id = rank of the representative among representatives; offsets into the factor tables (class * nwl).  A
+    // node's record holds its position ls and its phase / depth offsets (as the low / high word of the second double), so
+    // the walks fetch everything a node step needs from the plan with one 16-byte load
     for (int j = tid; j < Ns; j += T) {
         const int rw = iscr[j], rh = iscr[NsP + j];
         int wi = -1, hi = -1;
@@ -156,10 +158,13 @@ __global__ void __launch_bounds__(128) k_fused_plan(DesignsDev D, double *plan, 
         if (hi >= maxH) { hi = 0; cnt[2] = 1; }
         if (rw == j && wi >= 0) { wkey[2 * wi] = scr[j]; wkey[2 * wi + 1] = scr[NsP + j]; atomicMax(&cnt[0], wi + 1); }
         if (rh == j && hi >= 0) { hkey[hi] = scr[2 * NsP + j]; atomicMax(&cnt[1], hi + 1); }
-        node_w[j] = (wi >= 0 ? wi : maxW) * nwl;             // identity row when the phase / depth does not change
-        node_h[j] = (hi >= 0 ? hi : maxH) * nwl;
+        // identity row when the phase / depth does not change
+        rec[j] = make_double2(D.node_ls[nbase + j], __hiloint2double((hi >= 0 ? hi : maxH) * nwl, (wi >= 0 ? wi : maxW) * nwl));
     }
-    for (int j = Ns + tid; j < NsP + 12; j += T) { node_w[j] = maxW * nwl; node_h[j] = maxH * nwl; node_m[j] = Nm > 0 ? Nm - 1 : 0; }
+    for (int j = Ns + tid; j < NsP + 12; j += T) {
+        rec[j] = make_double2(0.0, __hiloint2double(maxH * nwl, maxW * nwl));
+        node_m[j] = Nm > 0 ? Nm - 1 : 0;
+    }
     // z classes of the members' first nodes
     for (int m = tid; m < Nm; m += T) {
         const double z0 = z0s[m];
@@ -288,6 +293,10 @@ __device__ __forceinline__ bool conv_ok(double dr, double di, double xr, double 
     return a < rhs * rhs;
 }
 
+// FULL = false: the instantiation for calls without BEM added mass / damping tables (A_w, B_w), F_drag or Xi_last outputs
+// and without the primary-case hand-over (lin_g); those paths are compiled out of its pass loop, which keeps the loop's
+// code (instruction-cache footprint) smaller.  The host selects it from the inputs (run_fused2 in raftk.cu).
+template <bool FULL>
 __global__ void __launch_bounds__(F2_T, 2)
 k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
 {
@@ -301,7 +310,7 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
     const int unit = blockIdx.x / CS;
     const int d = unit / Cs.nC, c = unit % Cs.nC;
     const int nw = D.nw, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int prim = (P.phase >= 0 && Cs.primary) ? Cs.primary[c] : c;
+    const int prim = (FULL && P.phase >= 0 && Cs.primary) ? Cs.primary[c] : c;
     const bool secondary = prim != c;
     if ((P.phase == 0 && secondary) || (P.phase == 1 && !secondary)) return;
 
@@ -316,7 +325,10 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
     double *s_mem = blob + L.o_mem, *s_node = blob + L.o_node, *s_mat = blob + L.o_mat;
     const double *s_wkey = blob + L.o_wkey, *s_hkey = blob + L.o_hkey, *s_zkey = blob + L.o_zkey;
     const int *ib = reinterpret_cast<const int *>(blob + L.o_int);
-    const int *s_imem = ib + L.i_imem, *s_nodew = ib + L.i_nodew, *s_nodeh = ib + L.i_nodeh, *s_nodem = ib + L.i_nodem, *s_cnt = ib + L.i_cnt;
+    const int *s_imem = ib + L.i_imem, *s_nodem = ib + L.i_nodem, *s_cnt = ib + L.i_cnt;
+    const double2 *s_rec = reinterpret_cast<const double2 *>(blob + L.o_rec);  // per node: ls, factor-table offsets (F2_OW / F2_OH)
+#define F2_OW(R) __double2loint((R).y)
+#define F2_OH(R) __double2hiint((R).y)
     const int *s_chunk = ib + L.i_chunk;
     double *p = blob + L.total;
     double *s_coef = p; p += NCOEF * (size_t)NsP;
@@ -444,8 +456,8 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
             double AqrA = 0, AqiA = 0, A1rA = 0, A1iA = 0, A2rA = 0, A2iA = 0, L1rA = 0, L1iA = 0, L2rA = 0, L2iA = 0;
             double AqrB = 0, AqiB = 0, A1rB = 0, A1iB = 0, A2rB = 0, A2iB = 0, L1rB = 0, L1iB = 0, L2rB = 0, L2iB = 0;
             for (int j = j0; j < j1; j++) {
-                const int ow = s_nodew[j], oh = s_nodeh[j];
-                const double2 WA = wtA[ow], HA = htA[oh], WB = wtB[ow], HB = htB[oh];
+                const double2 rj = s_rec[j];
+                const double2 WA = wtA[F2_OW(rj)], HA = htA[F2_OH(rj)], WB = wtB[F2_OW(rj)], HB = htB[F2_OH(rj)];
                 { const double tr = fma(erA, WA.x, -eiA * WA.y); eiA = fma(erA, WA.y, eiA * WA.x); erA = tr; }
                 { const double tr = fma(erB, WB.x, -eiB * WB.y); eiB = fma(erB, WB.y, eiB * WB.x); erB = tr; }
                 apA *= HA.x; amA *= HA.y; apB *= HB.x; amB *= HB.y;
@@ -529,8 +541,8 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
     }
     __syncthreads();
 
-    const double *Aw = D.A_w ? D.A_w + (size_t)d * 36 * nw : nullptr;
-    const double *Bw = D.B_w ? D.B_w + (size_t)d * 36 * nw : nullptr;
+    const double *Aw = FULL && D.A_w ? D.A_w + (size_t)d * 36 * nw : nullptr;
+    const double *Bw = FULL && D.B_w ? D.B_w + (size_t)d * 36 * nw : nullptr;
     int passes = 0, converged = 0, flags = plan_overflow ? RAFTK_FLAG_PLAN : 0, par = 0;
     const int max_pass = plan_overflow ? 0 : (secondary ? 1 : P.n_iter + 1);
     const size_t lin_stride = (size_t)NCOEF * NsP + 36;
@@ -612,8 +624,8 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
 #define F2_P1_NODE(JJ, CWA, CHA, CWB, CHB, CL, NWA, NHA, NWB, NHB, NL)                                                           \
     {                                                                                                                             \
         const int jn = jc0 + JJ + 1;                                                                                              \
-        const int ow = s_nodew[jn], oh = s_nodeh[jn];                                                                             \
-        NWA = wtA[ow]; NHA = htA[oh]; NWB = wtB[ow]; NHB = htB[oh]; NL = n_ls[jn];                                                \
+        const double2 rn = s_rec[jn];                                                                                             \
+        NWA = wtA[F2_OW(rn)]; NHA = htA[F2_OH(rn)]; NWB = wtB[F2_OW(rn)]; NHB = htB[F2_OH(rn)]; NL = rn.x;                        \
         const double ls = CL;                                                                                                     \
         F2_STEP_BIN(erA, eiA, apA, amA, CWA, CHA, CcA, ScA)                                                                       \
         F2_STEP_BIN(erB, eiB, apB, amB, CWB, CHB, CcB, ScB)                                                                       \
@@ -635,8 +647,8 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
     }
                     double2 WaA, HaA, WaB, HaB, WbA, HbA, WbB, HbB; double La, Lb;
                     {
-                        const int ow = s_nodew[jfirst], oh = s_nodeh[jfirst];
-                        WaA = wtA[ow]; HaA = htA[oh]; WaB = wtB[ow]; HaB = htB[oh]; La = n_ls[jfirst];
+                        const double2 rf = s_rec[jfirst];
+                        WaA = wtA[F2_OW(rf)]; HaA = htA[F2_OH(rf)]; WaB = wtB[F2_OW(rf)]; HaB = htB[F2_OH(rf)]; La = rf.x;
                         WbA = WaA; HbA = HaA; WbB = WaB; HbB = HaB; Lb = La;
                     }
                     switch (jj) {
@@ -750,7 +762,7 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
             if (P.Bdrag_out && rank == 0) P.Bdrag_out[((size_t)d * Cs.nC + c) * 36 + tid] = s;
         }
         __syncthreads();
-        if (P.lin_g && P.phase == 0 && rank == 0) {
+        if (FULL && P.lin_g && P.phase == 0 && rank == 0) {
             double *dst = P.lin_g + ((size_t)d * Cs.nC + c) * lin_stride;
 #pragma unroll 1
             for (int t = tid; t < NCOEF * NsP; t += T) dst[t] = s_coef[t];
@@ -783,8 +795,8 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
                 double AqrB = 0, AqiB = 0, A1rB = 0, A1iB = 0, A2rB = 0, A2iB = 0, L1rB = 0, L1iB = 0, L2rB = 0, L2iB = 0;
 #pragma unroll 2
                 for (int j = j0; j < j1; j++) {
-                    const int ow = s_nodew[j], oh = s_nodeh[j];
-                    const double2 WA = wtA[ow], HA = htA[oh], WB = wtB[ow], HB = htB[oh];
+                    const double2 rj = s_rec[j];
+                    const double2 WA = wtA[F2_OW(rj)], HA = htA[F2_OH(rj)], WB = wtB[F2_OW(rj)], HB = htB[F2_OH(rj)];
                     const double bq = cq_[j], b1 = c1_[j], lb1 = cl1_[j], b2 = c2_[j], lb2 = cl2_[j];
                     { const double tr = fma(erA, WA.x, -eiA * WA.y); eiA = fma(erA, WA.y, eiA * WA.x); erA = tr; }
                     { const double tr = fma(erB, WB.x, -eiB * WB.y); eiB = fma(erB, WB.y, eiB * WB.x); erB = tr; }
@@ -839,7 +851,7 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
 #pragma unroll
                 for (int a = 0; a < 6; a++) { const double2 v = P.Xi_out[ogl + (size_t)a * nw + i]; br[a] = v.x; bi[a] = v.y; }
             }
-            if (P.Fdrag_out) {
+            if (FULL && P.Fdrag_out) {
 #pragma unroll
                 for (int a = 0; a < 6; a++) P.Fdrag_out[ogl + (size_t)a * nw + i] = make_double2(br[a], bi[a]);
             }
@@ -879,7 +891,7 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
                 s_xi[(2 * a) * nwl + t] = 0.2 * lr + 0.8 * br[a];
                 s_xi[(2 * a + 1) * nwl + t] = 0.2 * li + 0.8 * bi[a];
                 P.Xi_out[ogl + (size_t)a * nw + i] = make_double2(br[a], bi[a]);
-                if (P.Xilast_out) P.Xilast_out[ogl + (size_t)a * nw + i] = make_double2(lr, li);
+                if (FULL && P.Xilast_out) P.Xilast_out[ogl + (size_t)a * nw + i] = make_double2(lr, li);
             }
         }
         passes++;
@@ -917,6 +929,8 @@ k_rao_fused2(DesignsDev D, CasesDev Cs, FusedParams P)
         if (nan_all & RAFTK_FLAG_NAN) break;
         if (conv_all) { converged = 1; break; }
     }
+#undef F2_OW
+#undef F2_OH
     if (P.status && rank == 0 && tid == 0) {
         int *st = P.status + ((size_t)d * Cs.nC + c) * 4;
         st[0] = secondary ? 0 : passes; st[1] = secondary ? 1 : converged; st[2] = flags; st[3] = secondary ? prim + 1 : 0;
